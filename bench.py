@@ -5,6 +5,7 @@
     python bench.py --workload llama_prefill --steps 10 --warmup 3      # tokens/s, LLaMA-7B prefill, S=2048
     python bench.py --impl reference ...                                 # the reference algorithm on the host CPU
     torchrun --nproc-per-node N ... bench.py --gpus N ...                # one rank per GPU, weak scaling
+    python bench.py ... --dump-outputs DIR                               # + the last timed step's outputs as .npy
 
 One "step" is one pass of the hot path over one batch of synthetic input:
   encode        : 256 images/GPU -> [256,32] ids (config #2 of BASELINE.json); at N > 1 every rank encodes its own
@@ -16,6 +17,11 @@ With the default workload the line also carries `secondary` records for the LLaM
 reference-facing Python API (models.seed_llama_tokenizer.ImageTokenizer.encode / models.llama_xformer
 .LlamaForCausalLM.forward) starting from PINNED HOST buffers and ending with the ids / last-token logits on
 the host, copies inside the timed region.  Prints ONE JSON line on rank 0.
+
+--dump-outputs DIR writes, on rank 0, what each arm's timed path returned in its last timed step as DIR/<name>.npy
+(integer outputs such as ids as float64, which holds them exactly, the rest as float32; at most 64 MB in all).  Inputs
+and weights are seeded, so two builds run with the same arguments can be compared output for output.  Outputs too
+large to keep whole are a fixed seeded sample: 64 positions of the prefill logits, 16 images of the preprocess batch.
 """
 from __future__ import annotations
 
@@ -32,6 +38,7 @@ import torch
 REPO = os.path.dirname(os.path.abspath(__file__))
 if REPO not in sys.path:
     sys.path.insert(0, REPO)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (no __pycache__)
 
 VIT_DEPTH, QF_LAYERS = 39, 12
 # algorithmic work per image (2 FLOP per MAC), SURVEY.md section 8d / DESIGN.md
@@ -157,6 +164,35 @@ def timed(fn, steps, warmup, world):
     barrier_sync(world)
     LAST_LOCAL_MS[0] = s.elapsed_time(e)
     return max_over_ranks(LAST_LOCAL_MS[0], world)
+
+
+OUTPUTS = {}                    # --dump-outputs: name -> host array of the last timed step
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def keep_outputs(**tensors):
+    """host copies of the last timed step's outputs, taken right after the timed region (the e2e and profiling calls
+    that follow may reuse the buffers the outputs live in)"""
+    for name, t in tensors.items():
+        t = t.detach().cpu()
+        OUTPUTS[name] = (t.float() if t.is_floating_point() else t.double()).numpy()
+
+
+def seeded_rows(n: int, k: int) -> torch.Tensor:
+    """a fixed sample of min(k, n) of n row indices, sorted: the same rows on every run of every build"""
+    return torch.randperm(n, generator=torch.Generator().manual_seed(0))[:k].sort().values
+
+
+def write_outputs(directory: str) -> None:
+    import numpy as np
+
+    total = sum(a.nbytes for a in OUTPUTS.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: outputs of {total / 2**20:.1f} MB exceed the {DUMP_LIMIT_BYTES >> 20} MB of "
+                         "--dump-outputs; use a smaller --batch")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in OUTPUTS.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def workload_config(args, world):
@@ -402,6 +438,8 @@ def encode_arm(args, world, rank, local, keep=None):
     L.reset_launch_count()
     with ClockSampler(local) as cs:
         ms = timed(step_device, args.steps, args.warmup, world)
+    if args.dump_outputs:
+        keep_outputs(encode_ids=out["ids"])
     rank_ms = per_rank_stats(LAST_LOCAL_MS[0] / args.steps, world)
     launches = L.launch_count() // (args.steps + args.warmup)
     clocks = cs.summary()
@@ -511,6 +549,8 @@ def llama_decode_arm(args, world, rank, local):
     L.reset_launch_count()
     with ClockSampler(local) as cs:
         ms = timed(step_device, args.steps, args.warmup, world)
+    if args.dump_outputs:
+        keep_outputs(llama_decode_sequence=out["seq"])
     rank_ms = per_rank_stats(LAST_LOCAL_MS[0] / args.steps, world)
     launches = L.launch_count() // (args.steps + args.warmup)
     clocks = cs.summary()
@@ -583,6 +623,8 @@ def preprocess_arm(args, world, rank, local):
     L.reset_launch_count()
     with ClockSampler(local) as cs:
         ms = timed(step_device, args.steps, args.warmup, world)
+    if args.dump_outputs:
+        keep_outputs(preprocess_pixels_sample=out["y"][seeded_rows(B, 16).to(dev)])
     launches = L.launch_count() // (args.steps + args.warmup)
     clocks = cs.summary()
     ms_e2e = timed(step_e2e, args.steps, max(1, args.warmup), world)
@@ -642,6 +684,8 @@ def llama_arm(args, world, rank, local, keep=None):
     L.reset_launch_count()
     with ClockSampler(local) as cs:
         ms = timed(step_device, args.steps, args.warmup, world)
+    if args.dump_outputs:
+        keep_outputs(llama_prefill_logits_sample=out["o"].logits[0, seeded_rows(S, 64).to(dev)])
     rank_ms = per_rank_stats(LAST_LOCAL_MS[0] / args.steps, world)
     launches = L.launch_count() // (args.steps + args.warmup)
     clocks = cs.summary()
@@ -724,6 +768,8 @@ def pipeline_arm(args, world, rank, local, tok=None, model=None):
     L.reset_launch_count()
     with ClockSampler(local) as cs:
         ms = timed(step_device, args.steps, args.warmup, world)
+    if args.dump_outputs:
+        keep_outputs(pipeline_last_logits=out["o"].logits)
     rank_ms = per_rank_stats(LAST_LOCAL_MS[0] / args.steps, world)
     launches = L.launch_count() // (args.steps + args.warmup)
     clocks = cs.summary()
@@ -782,7 +828,13 @@ def main():
     ap.add_argument("--no-secondary", action="store_true",
                     help="encode workload only: skip the LLaMA half of BASELINE.json's metric (secondary records)")
     ap.add_argument("--ref-seconds", type=float, default=150.0, help="wall-clock budget of the --impl reference run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step of every arm as DIR/<name>.npy (seedb200 arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the seedb200 arm")
     args.warmup = max(args.warmup, 3) if args.impl == "seedb200" else args.warmup
 
     if args.impl == "reference":
@@ -843,6 +895,8 @@ def main():
         dist.barrier()
         dist.destroy_process_group()
     if rank == 0:
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs)
         print(json.dumps(res), flush=True)
 
 

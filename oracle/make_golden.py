@@ -69,6 +69,26 @@ def encoder_golden(name: str, vit_depth: int, qformer_layers: int, detok_depth: 
           f"({time.time() - t0:.0f}s)")
 
 
+def encoder_fresh_seed_golden(name: str = "encoder_v1_q2_d1_seed77.pt") -> None:
+    """get_codebook_indices / get_codebook_entry outputs on weights and images of other seeds than the files above,
+    with a de-tokenizer block: 1 ViT block, 2 Q-Former layers, 1 de-tokenizer block, 2 images."""
+    vd, ql, dd, batch, wseed, iseed = 1, 2, 1, 2, 77, 78
+    model = ref_shim.build_reference_quantizer(vd, ql, dd)
+    model.load_state_dict(synth.encoder_state_dict(vd, ql, dd, seed=wseed), strict=False)
+    x = synth.images(batch, seed=iseed)
+    with torch.no_grad():
+        ids, query_up = model.get_codebook_indices(x)
+        embeds = model.get_codebook_entry(ids)
+    out = {
+        "config": {"vit_depth": vd, "qformer_layers": ql, "detok_depth": dd, "batch": batch, "weights_seed": wseed,
+                   "images_seed": iseed, "dtype": "fp32 (reference CPU mode)",
+                   "reference": "models/seed_qformer/qformer_quantizer.py get_codebook_indices/get_codebook_entry"},
+        "ids": ids.clone(), "query_output_up": query_up.clone(), "image_embeds_out": embeds.clone(),
+    }
+    torch.save(out, os.path.join(GOLDEN_DIR, name))
+    print(f"{name}: ids[0,:8]={ids[0, :8].tolist()} query_output_up {tuple(query_up.shape)}")
+
+
 def llama_golden(name: str = "llama_tiny.pt") -> None:
     L = ref_shim.load_llama_module()
     from transformers.models.llama.configuration_llama import LlamaConfig
@@ -97,23 +117,37 @@ def llama_golden(name: str = "llama_tiny.pt") -> None:
     print(f"{name}: logits {tuple(out.logits.shape)} next {nxt.flatten().tolist()}")
 
 
+VQ_CASES = {"spread": (512, 0.28, 99), "default_init": (128, None, 98)}       # rows of z, codebook std, seed
+
+
+def vq_inputs(tag: str) -> tuple[torch.Tensor, torch.Tensor]:
+    """z [n,32] and the 8192 x 32 codebook (both fp16) of VQ case `tag`.  The codebooks are drawn here rather than
+    stored (512 KB each); vq_golden keeps a strided sample of each so that a changed draw is caught."""
+    n, cstd, seed = VQ_CASES[tag]
+    g = torch.Generator().manual_seed(seed)
+    z = (torch.randn(n, 32, generator=g) * 0.28).half()
+    if cstd is None:    # the reference's default init, U(-1/n_e, 1/n_e) (qformer_quantizer.py:39)
+        cb = (torch.rand(8192, 32, generator=g, dtype=torch.float64) * 2 - 1) / 8192
+    else:
+        cb = torch.randn(8192, 32, generator=g) * cstd
+    return z, cb.half()
+
+
 def vq_golden(name: str = "vq_reference_expr.pt") -> None:
     """The reference distance/argmin expression itself (qformer_quantizer.py:94-98) in fp32 and in half."""
     qq = ref_shim.load_quantizer_module()
-    g = torch.Generator().manual_seed(99)
     res = {}
-    for tag, n, n_codes, cstd in (("spread", 512, 8192, 0.28), ("default_init", 128, 8192, None)):
-        z = (torch.randn(n, 32, generator=g) * 0.28).half()
+    for tag in VQ_CASES:
+        z, cb = vq_inputs(tag)
+        n, n_codes = z.shape[0], cb.shape[0]
         vq = qq.VectorQuantizer2(n_codes, 32, beta=0.25)
-        if cstd is not None:
-            vq.embedding.weight.data = (torch.randn(n_codes, 32, generator=g) * cstd)
-        vq.embedding.weight.data = vq.embedding.weight.data.half().float()
-        cb = vq.embedding.weight.data.half()
+        vq.embedding.weight.data = cb.float()
         with torch.no_grad():
             _, _, ids32 = vq(z.float().view(n // 32, 32, 32))
             vq16 = vq.half()
             _, _, ids16 = vq16(z.view(n // 32, 32, 32))
-        res[tag] = {"z": z, "codebook": cb, "ids_fp32": ids32.flatten().clone(), "ids_fp16": ids16.flatten().clone()}
+        res[tag] = {"z": z, "codebook_sample": _sample(cb), "ids_fp32": ids32.flatten().clone(),
+                    "ids_fp16": ids16.flatten().clone()}
         print(f"{name}/{tag}: fp32 vs fp16 agreement {(ids32 == ids16).float().mean():.4f}")
     torch.save(res, os.path.join(GOLDEN_DIR, name))
 
@@ -124,6 +158,7 @@ def main() -> None:
     vq_golden()
     llama_golden()
     encoder_golden("encoder_d2_q2.pt", 2, 2, 1, 2)
+    encoder_fresh_seed_golden()
     if "--full" in sys.argv:
         encoder_golden("encoder_full.pt", 39, 12, 4, 2)
 

@@ -4,8 +4,7 @@ The reference pins transformers 4.30 / timm / xformers / diffusers, none of whic
 module registers ~40 lines of stub modules and back-fills three removed transformers helpers so that
 `models.seed_qformer.qformer_quantizer` and `models.llama_xformer` import and run as shipped (recipe and
 probes: SURVEY.md section 8c).  It exists only in the build container (the GPU box has no /root/reference);
-it is used by oracle/make_golden.py to generate tests/golden/* and by tests that pin oracle/restatement.py
-against the real reference when it is available.
+it is used by oracle/make_golden.py to generate tests/golden/*, which the tests compare against.
 
 Nothing here is arithmetic: the stubs replace (a) timm init helpers (trunc_normal_, to_2tuple, DropPath),
 (b) three network-touching factories (BertTokenizer / BertLMHeadModel.from_pretrained / eva_vit_g.pth

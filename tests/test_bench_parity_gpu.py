@@ -5,10 +5,9 @@
 * the reference's *GPU* mode (`fp16: True`: `model.half()`, ViT + ln_vision under CUDA autocast, the rest in plain fp16 --
   models/seed_llama_tokenizer.py:58-59,86-87, qformer_quantizer.py:288-307) restated with torch on the GPU box as a
   second oracle (SURVEY.md section 8c): how far that mode sits from fp32, how far this build sits from fp32, and the
-  id agreement between all three.  The numbers are written to gpurun_out/r02_autocast_oracle.json.
+  id agreement between all three.  The numbers are printed as one JSON line.
 """
 import json
-import os
 
 import pytest
 import torch
@@ -100,11 +99,6 @@ def test_reference_gpu_mode_as_a_second_oracle(full):
         "note": "reference GPU mode = model.half(), ViT + ln_vision under torch.autocast(fp16), Q-Former / heads / VQ in "
                 "plain fp16 (restated with torch on this GPU); fp32 oracle = oracle/restatement.py on the host",
     }
-    try:
-        os.makedirs("gpurun_out", exist_ok=True)
-        json.dump(report, open("gpurun_out/r02_autocast_oracle.json", "w"), indent=1)
-    except OSError:
-        pass
     print(json.dumps(report))
     # this build keeps scores / statistics / accumulators in fp32 where the reference's GPU mode rounds to fp16: it
     # must sit at least as close to the fp32 oracle as that mode does (with slack for rounding noise)

@@ -1,7 +1,6 @@
-"""CPU tests (-m "not gpu") that PIN the oracle:
-  * oracle/restatement.py (plain-torch restatement) and oracle/vq_oracle.c (C restatement of the VQ search)
-    against tests/golden/*.pt, which oracle/make_golden.py produced by running the unmodified reference;
-  * and, when /root/reference is mounted (build container only), against the live reference itself.
+"""CPU tests (-m "not gpu") that PIN the oracle: oracle/restatement.py (plain-torch restatement) and
+oracle/vq_oracle.c (C restatement of the VQ search) against tests/golden/*.pt, which oracle/make_golden.py
+produced by running the unmodified reference.
 """
 import ctypes as C
 import os
@@ -10,7 +9,8 @@ import numpy as np
 import pytest
 import torch
 
-from oracle import ref_shim, restatement as R, synth
+from oracle import restatement as R, synth
+from oracle.make_golden import vq_inputs
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -54,8 +54,12 @@ def c_oracle(lib, z16, cb16, mode):
 @pytest.mark.parametrize("tag", ["spread", "default_init"])
 def test_c_vq_oracle_matches_reference_vectors(vq_lib, tag):
     g = _load("vq_reference_expr.pt")[tag]
-    ids32, m32 = c_oracle(vq_lib, g["z"], g["codebook"], 1)
-    ids16, m16 = c_oracle(vq_lib, g["z"], g["codebook"], 0)
+    z, cb = vq_inputs(tag)
+    s = g["codebook_sample"]
+    assert torch.equal(z, g["z"]) and list(cb.shape) == s["shape"]
+    assert torch.equal(cb.reshape(-1)[:: s["step"]], s["values"])        # the codebook is the one the ids came from
+    ids32, m32 = c_oracle(vq_lib, z, cb, 1)
+    ids16, m16 = c_oracle(vq_lib, z, cb, 0)
     # exact wherever the oracle's own top-2 margin is not a floating-point tie; report would-be flips
     neq32 = ids32 != g["ids_fp32"]
     neq16 = ids16 != g["ids_fp16"]
@@ -112,21 +116,20 @@ def test_encoder_restatement_matches_golden_full_depth():
     _encoder_vs_golden("encoder_full.pt")
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="/root/reference not mounted (GPU box)")
-def test_encoder_restatement_matches_live_reference():
-    vd, ql, dd = 1, 2, 1
-    model = ref_shim.build_reference_quantizer(vd, ql, dd)
-    sd = synth.encoder_state_dict(vd, ql, dd, seed=77)
-    model.load_state_dict(sd, strict=False)
-    x = synth.images(2, seed=78)
+def test_encoder_restatement_matches_reference_on_fresh_seeds():
+    """the reference's get_codebook_indices / get_codebook_entry outputs on other weight and image seeds, with a
+    de-tokenizer block (tests/golden/encoder_v1_q2_d1_seed77.pt)"""
+    g = _load("encoder_v1_q2_d1_seed77.pt")
+    c = g["config"]
+    vd, ql, dd = c["vit_depth"], c["qformer_layers"], c["detok_depth"]
+    sd = synth.encoder_state_dict(vd, ql, dd, seed=c["weights_seed"])
+    x = synth.images(c["batch"], seed=c["images_seed"])
     with torch.no_grad():
-        ids, up = model.get_codebook_indices(x)
-        emb = model.get_codebook_entry(ids)
         out = R.encode(x, sd, vd, ql)
-        emb2 = R.detokenize(ids, sd, dd)
-    assert torch.equal(ids, out["ids"])
-    assert torch.allclose(up, out["query_output_up"], atol=1e-5)
-    assert torch.allclose(emb, emb2, atol=1e-5)
+        emb2 = R.detokenize(g["ids"], sd, dd)
+    assert torch.equal(g["ids"], out["ids"])
+    assert torch.allclose(g["query_output_up"], out["query_output_up"], atol=1e-5)
+    assert torch.allclose(g["image_embeds_out"], emb2, atol=1e-5)
 
 
 # ---------------------------------------------------------------------------------------------
